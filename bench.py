@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the RoIAlign hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input at BASELINE.json configs[1]:
 RoIAlign (Caffe2-exact) forward + backward, 1x256x200x272 fp32 feature map, 512 RoIs, 7x7, sr=2.
@@ -15,6 +15,10 @@ Keys beyond the base contract:
   e2e           same metric through the reference-shaped plugin with HOST buffers (H2D + D2H timed)
   kernels       per-kernel launch times / fractions, plus the reference's own CUDA kernels
                 (oracle/_ref, recompiled for sm_100a) timed on the same inputs when present
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) as float32 .npy files: roi_align_out.npy, the
+whole forward output (512, 256, 7, 7), and grad_features_even_channels.npy, the feature-map gradient of every second
+channel (1, 128, 200, 272) -- 53.5 MB in all.  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 `--impl reference` times the reference algorithm on the host cores (the reference has no CPU
 RoIAlign -- functions/roi_align.py:28-29 -- so this is the op-for-op C restatement in oracle/).
 """
@@ -42,7 +46,13 @@ def parse_args():
     ap.add_argument("--sets", type=int, default=6, help="rotating input sets (each 163 MB) so no step re-reads L2-resident data")
     ap.add_argument("--no-graph", action="store_true", help="time direct launches instead of a CUDA graph of the K steps")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
+    return args
 
 
 def load_peaks():
@@ -153,7 +163,7 @@ def main():
     cfg = S.CFG2
     shape, P, scale, sr, R = cfg["shape"], cfg["pooled"], cfg["scale"], cfg["sampling_ratio"], cfg["rois"]
     N, C, H, W = shape
-    K, Wm = max(1, args.steps), max(3, args.warmup)
+    K, Wm = args.steps, max(3, args.warmup)
     nsets = max(2, args.sets)
 
     # ---- synthetic inputs, resident in HBM; `nsets` independent sets are rotated so that every step
@@ -235,6 +245,9 @@ def main():
             sys.stderr.write("bench: CUDA graph path failed (%s); timing direct launches\n" % exc)
             use_graph = False
             ms_total = timed(step, K, graph=False)
+        # the timed steps were 0 .. K-1: keep what the last one wrote before anything else runs on these buffers
+        last = (K - 1) % nsets
+        dumped = (outs[last].clone(), dxs[last][:, ::2].clone()) if args.dump_outputs and rank == 0 else None
         # The timed region is only ~35 ms long (nvidia-smi samples every 100 ms): keep replaying the identical steps,
         # untimed, for another half second so that the clock / throttle samples are taken under this very load.
         t_soak = time.perf_counter()
@@ -374,6 +387,10 @@ def main():
             "clocks": clocks, "kernels": kernels,
         }
         print(json.dumps(line))
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in zip(("roi_align_out", "grad_features_even_channels"), dumped):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy().astype(np.float32))
     if world > 1:
         dist.destroy_process_group()
     return 0

@@ -25,6 +25,46 @@ def roi_case(name):
     return c, feats, rois, dy
 
 
+def sample_index(size, seed, k=8192):
+    """A fixed, seeded sample of k flat indices into an array of `size` elements: large outputs are stored under
+    tests/golden/ as their values at these indices."""
+    return np.sort(np.random.RandomState(seed).choice(size, k, replace=False))
+
+
+def spread_cases():
+    """name -> (shape, scale, P, sr, rois, dy seed): the backward run-to-run spread cases (BASELINE cfg2 and a pile-up)."""
+    return {
+        "cfg2": (S.CFG2["shape"], S.CFG2["scale"], S.CFG2["pooled"], S.CFG2["sampling_ratio"],
+                 S.make_rois(S.CFG2["rois"], S.CFG2["shape"], S.CFG2["scale"]).astype(np.float32), 1),
+        "pileup_1500": ((3, 40, 46, 70), 0.125, 7, 2,
+                        S.make_rois(1500, (3, 40, 46, 70), 0.125, seed=6, min_size=64, max_size=500).astype(np.float32), 7),
+    }
+
+
+# (soft_nms, soft_method, bbox_vote, vote_scoring) settings of the test-time detection post-processing
+DETECTION_SETTINGS = (
+    (False, "linear", False, "ID"), (True, "linear", False, "ID"), (True, "gaussian", False, "ID"),
+    (False, "linear", True, "ID"), (False, "linear", True, "IOU_AVG"), (True, "linear", True, "AVG"),
+    (False, "linear", True, "TEMP_AVG"), (False, "linear", True, "QUASI_SUM"), (False, "linear", True, "GENERALIZED_AVG"),
+)
+
+
+def detection_case(seed, R=300, K=21):
+    """Clustered proposals: 25 objects x 12 jittered copies, every class gets its own regressed box per proposal.
+    Returns scores (R, K) and boxes (R, 4K), fp32."""
+    rng = np.random.RandomState(seed)
+    cx = np.repeat(rng.uniform(100, 1200, 25), 12)[:R]; cy = np.repeat(rng.uniform(100, 700, 25), 12)[:R]
+    w = np.repeat(rng.uniform(40, 300, 25), 12)[:R]; h = np.repeat(rng.uniform(40, 300, 25), 12)[:R]
+    boxes = np.zeros((R, 4 * K), np.float32)
+    for j in range(K):
+        jx = cx + rng.normal(0, 0.06, R) * w; jy = cy + rng.normal(0, 0.06, R) * h
+        jw = w * (1 + rng.normal(0, 0.08, R)); jh = h * (1 + rng.normal(0, 0.08, R))
+        boxes[:, 4 * j:4 * j + 4] = np.stack([jx - jw / 2, jy - jh / 2, jx + jw / 2, jy + jh / 2], 1)
+    logits = rng.standard_normal((R, K)) * 2.0
+    scores = (np.exp(logits) / np.exp(logits).sum(1, keepdims=True)).astype(np.float32)
+    return scores, boxes
+
+
 def crop_case(seed=0):
     shape = (2, 6, 30, 44)
     img = S.make_features(shape, seed=seed)

@@ -1,72 +1,43 @@
 """SURVEY.md 8f N3: test-time detection post-processing on the device (per-class NMS in one batched launch pair, soft-NMS,
 box voting, the per-image limit) against the REFERENCE'S OWN functions -- lib/core/test.py:732-790, lib/utils/boxes.py and
-the Cython routines built from its .pyx -- imported unmodified from oracle/_ref/reflib.  Runs in a subprocess: the
-reference's top-level packages (`utils`, `core`, `modeling`) must not leak into the other tests' sys.modules."""
+the Cython routines built from its .pyx.  Their results on the seeded inputs of tests/cases.py are stored in
+tests/golden/detections.npz (tests/golden/make_golden_detections.py runs the unmodified reference on CPU)."""
 import os
-import subprocess
-import sys
 
+import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from tests import cases
 
-CODE = r'''
-import sys, numpy as np, torch
-sys.path.insert(0, %r)
-from oracle import refmodel
-cfg = refmodel.setup(use_b200_ops=False)
-import core.test as ref_test
-from detectron.pytorch_b200.core.test import box_results_with_nms_and_limit as ours
-
-def make(seed, R=300, K=21):
-    rng = np.random.RandomState(seed)
-    # clustered proposals: 25 objects x 12 jittered copies, every class gets its own regressed box per proposal
-    cx = np.repeat(rng.uniform(100, 1200, 25), 12)[:R]; cy = np.repeat(rng.uniform(100, 700, 25), 12)[:R]
-    w = np.repeat(rng.uniform(40, 300, 25), 12)[:R]; h = np.repeat(rng.uniform(40, 300, 25), 12)[:R]
-    boxes = np.zeros((R, 4 * K), np.float32)
-    for j in range(K):
-        jx = cx + rng.normal(0, 0.06, R) * w; jy = cy + rng.normal(0, 0.06, R) * h
-        jw = w * (1 + rng.normal(0, 0.08, R)); jh = h * (1 + rng.normal(0, 0.08, R))
-        boxes[:, 4 * j:4 * j + 4] = np.stack([jx - jw / 2, jy - jh / 2, jx + jw / 2, jy + jh / 2], 1)
-    logits = rng.standard_normal((R, K)) * 2.0
-    scores = (np.exp(logits) / np.exp(logits).sum(1, keepdims=True)).astype(np.float32)
-    return scores, boxes
-
-cfg.MODEL.NUM_CLASSES = 21
-checked = 0
-for seed in (0, 1):
-    scores, boxes = make(seed)
-    for soft, method, vote, scoring in ((False, "linear", False, "ID"), (True, "linear", False, "ID"), (True, "gaussian", False, "ID"),
-                                        (False, "linear", True, "ID"), (False, "linear", True, "IOU_AVG"), (True, "linear", True, "AVG"),
-                                        (False, "linear", True, "TEMP_AVG"), (False, "linear", True, "QUASI_SUM"), (False, "linear", True, "GENERALIZED_AVG")):
-        cfg.TEST.SOFT_NMS.ENABLED = soft; cfg.TEST.SOFT_NMS.METHOD = method
-        cfg.TEST.BBOX_VOTE.ENABLED = vote; cfg.TEST.BBOX_VOTE.SCORING_METHOD = scoring; cfg.TEST.BBOX_VOTE.VOTE_TH = 0.8
-        cfg.TEST.SCORE_THRESH = 0.05; cfg.TEST.NMS = 0.5; cfg.TEST.DETECTIONS_PER_IM = 100
-        rs, rb, rc = ref_test.box_results_with_nms_and_limit(scores, boxes)
-        os_, ob, oc = ours(scores, boxes, cfg=cfg)
-        assert len(rc) == len(oc)
-        for j in range(1, 21):
-            a, b = np.asarray(rc[j]).reshape(-1, 5), np.asarray(oc[j]).reshape(-1, 5)
-            assert a.shape == b.shape, (seed, soft, method, vote, scoring, j, a.shape, b.shape)
-            if vote:      # numpy averages in float32 pairwise order; ours accumulates in fp64
-                np.testing.assert_allclose(b, a, rtol=1e-4, atol=2e-3)
-            elif soft and method == "gaussian":
-                np.testing.assert_allclose(b, a, rtol=1e-6, atol=1e-6)
-            else:
-                assert np.array_equal(a, b), (seed, soft, method, j)
-        assert rs.shape == os_.shape and rb.shape == ob.shape
-        checked += 1
-print("ok", checked)
-'''
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "detections.npz")
 
 
 @pytest.mark.gpu
 def test_box_results_with_nms_and_limit_matches_the_reference():
-    from oracle import refmodel
-    if not refmodel.available():
-        pytest.skip("oracle/_ref/reflib not built (python oracle/make_reflib.py in the build container)")
-    p = subprocess.run([sys.executable, "-c", CODE % ROOT], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
-    assert p.returncode == 0 and "ok 18" in p.stdout, (p.stdout[-1500:], p.stderr[-3000:])
+    from detectron.pytorch_b200.core.test import box_results_with_nms_and_limit as ours
+    g = np.load(GOLDEN)
+    checked = 0
+    for seed in (0, 1):
+        scores, boxes = cases.detection_case(seed)
+        for i, (soft, method, vote, scoring) in enumerate(cases.DETECTION_SETTINGS):
+            key = "%d_%d" % (seed, i)
+            os_, ob, oc = ours(scores, boxes, num_classes=21, score_thresh=0.05, nms=0.5, detections_per_im=100, soft_nms=soft,
+                               soft_sigma=float(g["soft_nms_sigma"]), soft_method=method, bbox_vote=vote, vote_th=0.8,
+                               vote_scoring=scoring)
+            assert len(oc) == 21
+            ref_cls = np.split(g[key + "/cls"], np.cumsum(g[key + "/cls_counts"])[:-1])
+            for j in range(1, 21):
+                a, b = ref_cls[j - 1], np.asarray(oc[j]).reshape(-1, 5)
+                assert a.shape == b.shape, (seed, soft, method, vote, scoring, j, a.shape, b.shape)
+                if vote:      # numpy averages in float32 pairwise order; ours accumulates in fp64
+                    np.testing.assert_allclose(b, a, rtol=1e-4, atol=2e-3)
+                elif soft and method == "gaussian":
+                    np.testing.assert_allclose(b, a, rtol=1e-6, atol=1e-6)
+                else:
+                    assert np.array_equal(a, b), (seed, soft, method, j)
+            assert g[key + "/scores"].shape == os_.shape and g[key + "/boxes"].shape == ob.shape
+            checked += 1
+    assert checked == 18
 
 
 def test_detection_batches_validate_on_the_host():
