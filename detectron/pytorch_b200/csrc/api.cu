@@ -54,9 +54,6 @@ void nms_set_timing_buffer(unsigned long long*);
 void roi_align_stream_set_debug_buffer(unsigned long long*);
 int roi_align_forward_tiled(const float*, float, int, int, int, int, int, int, int, int, const float*, float*, const int*, void*, size_t, cudaStream_t);
 size_t roi_align_stream_workspace_bytes(int, int, int, int, int, int, int);
-size_t roi_align_stream_fpn_workspace_bytes(int, const int*, const int*, int, int, int, int, int);
-int roi_align_forward_stream_fpn(int, const float* const*, const int*, const int*, const float*, const int*, int, int, int, int, int, int,
-                                 const float*, float*, const int*, void*, size_t, cudaStream_t);
 int roi_align_forward_stream(const float*, float, int, int, int, int, int, int, int, int, const float*, float*, const int*, void*, size_t, cudaStream_t);
 size_t roi_align_strip_workspace_bytes(int, int, int, int, int, int, int);
 size_t roi_align_strip_fpn_workspace_bytes(int, const int*, const int*, int, int, int, int, int);
@@ -411,16 +408,16 @@ int b200_nms(const float* boxes_dev, int boxes_num, int boxes_dim, float nms_ove
                workspace_bytes, (cudaStream_t)stream);
 }
 
+// The pyramid call runs the quad-strip path only, so its size is the only one that counts: 0 (the caller loops over the
+// levels) whenever that path would reject the geometry or the forward is forced onto another path.
 size_t b200_roi_align_fpn_workspace_bytes(int num_levels, const int* heights_host, const int* widths_host, int batch_size, int num_rois,
                                           int aligned_height, int aligned_width, int sampling_ratio) {
-    if (num_levels < 1 || !heights_host || !widths_host || batch_size <= 0 || num_rois <= 0 || forward_path_mode() == 1 || forward_path_mode() == 2 ||
+    const int mode = forward_path_mode();
+    if (num_levels < 1 || !heights_host || !widths_host || batch_size <= 0 || num_rois <= 0 || (mode != 0 && mode != 4) ||
         option_get(kOptFpnPath) == 'l')
         return 0;
-    const size_t a = roi_align_stream_fpn_workspace_bytes(num_levels, heights_host, widths_host, batch_size, num_rois, aligned_height,
-                                                          aligned_width, sampling_ratio);
-    const size_t b = forward_path_mode() == 3 ? 0 : roi_align_strip_fpn_workspace_bytes(num_levels, heights_host, widths_host, batch_size, num_rois,
-                                                                                        aligned_height, aligned_width, sampling_ratio);
-    return a > b ? a : b;
+    return roi_align_strip_fpn_workspace_bytes(num_levels, heights_host, widths_host, batch_size, num_rois, aligned_height, aligned_width,
+                                               sampling_ratio);
 }
 
 int b200_roi_align_forward_fpn(int num_levels, const float* const* bottom_data_host, const int* heights_host, const int* widths_host,
@@ -435,7 +432,8 @@ int b200_roi_align_forward_fpn(int num_levels, const float* const* bottom_data_h
     for (int l = 0; l < num_levels; ++l)
         if (!bottom_data_host[l] || level_roi_begin_host[l + 1] < level_roi_begin_host[l]) return B200_ROI_EINVAL;
     int rc = 1000;
-    if (forward_path_mode() != 3) {
+    const int mode = forward_path_mode();
+    if ((mode == 0 || mode == 4) && option_get(kOptFpnPath) != 'l') {
         // Levels that TMA can stage (W % 4 == 0, 16-byte aligned base) and levels that need the cp.async producers (FPN P5 of an
         // 800 x 1333 image: W = 42) go to separate launch sequences: runs of consecutive levels of the same kind, each over its
         // own contiguous range of the level-major RoIs.  The workspace is reused (stream order).

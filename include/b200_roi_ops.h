@@ -175,10 +175,12 @@ B200_API int b200_nms(const float* boxes_dev, int boxes_num, int boxes_dim, floa
  * RoIs of all levels stored level-major in bottom_rois (level l owns rows level_roi_begin_host[l] .. [l + 1]), and
  * top_rows[r] = the row of top_data RoI r is written to (the inverse of the reference's restore permutation; NULL:
  * identity).  The four *_host arrays and bottom_data_host (device pointers of the maps) are HOST arrays read during the
- * call.  One streaming kernel walks the strip columns of every level; results are bit-identical to per-level
- * b200_roi_align_forward calls.  b200_roi_align_fpn_workspace_bytes(...) == 0 means "not applicable" (sampling_ratio
- * outside {1, 2}, too many strip columns, path switched off): loop over b200_roi_align_forward_indexed instead;
- * b200_roi_align_forward_fpn then returns B200_ROI_EWORKSPACE. */
+ * call.  The quad-strip kernels walk the strip columns of every level; results are bit-identical to per-level
+ * b200_roi_align_forward calls.  This call has no fallback: b200_roi_align_fpn_workspace_bytes(...) is the quad-strip
+ * path's size alone, and it is 0 exactly when that path cannot run (sampling_ratio outside {1, 2}, PH or PW times
+ * sampling_ratio above 32, more than 96 strip columns or more than 6144 rows summed over them (all levels and images),
+ * more than 65535 RoIs, B200_ROI_ALIGN_PATH forced to generic / tiled / stream, B200_FPN_PATH=levels).  Then loop over
+ * b200_roi_align_forward_indexed instead; b200_roi_align_forward_fpn returns B200_ROI_EWORKSPACE. */
 B200_API size_t b200_roi_align_fpn_workspace_bytes(int num_levels, const int* heights_host, const int* widths_host,
                                                    int batch_size, int num_rois, int aligned_height, int aligned_width,
                                                    int sampling_ratio);

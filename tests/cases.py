@@ -12,6 +12,22 @@ ROI_CASES = {
     "sr3": dict(shape=(1, 4, 40, 40), scale=1.0 / 8, P=5, sr=3, n_rois=16),
 }
 
+PYRAMID_800x1333 = ((200, 336), (100, 168), (50, 84), (25, 42))        # (H, W) of FPN P2..P5 of an 800 x 1333 image
+
+# Both sides of every dispatch limit of the quad-strip forward (roi_align_strip.cu, strip_geometry), as
+# (N, H, W, R, PH, PW, sr).  Under B200_ROI_ALIGN_PATH=quad the single-map workspace size is the strip path's alone, so a
+# non-zero size means the path takes the shape.  tests/test_abi.py pins which side of each limit these shapes are on;
+# tests/test_gpu_geometry.py runs them on the GPU.
+QUAD_LIMITS = {
+    # limit: (accepted, rejected)
+    "keys_batch": ((16, 64, 336, 64, 7, 7, 2), (17, 64, 336, 64, 7, 7, 2)),          # 16 images x 6 strips x 64 rows = 6144 CSR keys
+    "keys_height": ((1, 1536, 100, 64, 7, 7, 2), (1, 1537, 100, 64, 7, 7, 2)),       # 4 strips x 1536 rows = 6144
+    "columns": ((1, 4, 5384, 64, 7, 7, 2), (1, 4, 5385, 64, 7, 7, 2)),              # 96 strips of one image
+    "rois": ((1, 50, 68, 65535, 7, 7, 2), (1, 50, 68, 65536, 7, 7, 2)),             # 16-bit RoI index of the fragment record
+    "axis_square": ((1, 50, 68, 64, 16, 16, 2), (1, 50, 68, 64, 17, 17, 2)),        # P * sr <= 32
+    "axis_pw": ((1, 50, 68, 64, 16, 3, 2), (1, 50, 68, 64, 3, 17, 2)),              # PH and PW are limited separately
+}
+
 NMS_SIZES = (1, 2, 63, 64, 65, 128, 129, 1000, 2000, 6000, 12000)
 
 

@@ -7,6 +7,7 @@ import re
 import pytest
 
 from detectron.pytorch_b200 import _lib, build
+from tests import cases
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -131,6 +132,49 @@ def test_round2_entry_points_validate_arguments_without_gpu():
     # single-map workspace covers the quad-strip path's tables, CSR records and temporary records
     w = lib.b200_roi_align_workspace_bytes(1, 512, 200, 272, 7, 7, 2)
     assert w >= 512 * 28 * 16 + 512 * 196 * 24
+
+
+def fpn_workspace_bytes(lib, levels, N, R, PH, PW, sr):
+    H = (ctypes.c_int * len(levels))(*[h for h, _ in levels]); W = (ctypes.c_int * len(levels))(*[w for _, w in levels])
+    return lib.b200_roi_align_fpn_workspace_bytes(len(levels), ctypes.cast(H, ctypes.c_void_p), ctypes.cast(W, ctypes.c_void_p),
+                                                  N, R, PH, PW, sr)
+
+
+@pytest.mark.parametrize("P,sr", [(7, 1), (7, 2), (14, 1), (14, 2), ((7, 14), 2)])
+def test_fpn_workspace_is_zero_exactly_when_the_pyramid_call_cannot_run(P, sr, lib_option):
+    """b200_roi_align_forward_fpn runs the quad-strip path only, so the size must be the strip path's alone: non-zero while the
+    pyramid fits the strip geometry (batch 1..5 of 800 x 1333 images), 0 from batch 6 on (too many strip columns / rows) and
+    whenever the forward is forced onto a path the pyramid call does not have.  A non-zero size there makes
+    RoIAlignFPNFunction call a forward that returns B200_ROI_EWORKSPACE instead of looping over the levels."""
+    lib = _lib.load()
+    PH, PW = P if isinstance(P, tuple) else (P, P)
+    sizes = [fpn_workspace_bytes(lib, cases.PYRAMID_800x1333, N, 1000, PH, PW, sr) for N in range(1, 9)]
+    assert all(s > 0 and s % 256 == 0 for s in sizes[:5]), sizes
+    assert sizes[5:] == [0, 0, 0], sizes
+    # forcing the quad-strip path changes nothing; forcing any other forward path, or the per-level loop, switches the call off
+    lib_option("B200_ROI_ALIGN_PATH", "quad")
+    assert fpn_workspace_bytes(lib, cases.PYRAMID_800x1333, 1, 1000, PH, PW, sr) == sizes[0]
+    assert fpn_workspace_bytes(lib, cases.PYRAMID_800x1333, 6, 1000, PH, PW, sr) == 0
+    for path in ("stream", "generic", "tiled"):
+        lib_option("B200_ROI_ALIGN_PATH", path)
+        assert [fpn_workspace_bytes(lib, cases.PYRAMID_800x1333, N, 1000, PH, PW, sr) for N in (1, 5, 8)] == [0, 0, 0], path
+    lib_option("B200_ROI_ALIGN_PATH", None)
+    lib_option("B200_FPN_PATH", "levels")
+    assert fpn_workspace_bytes(lib, cases.PYRAMID_800x1333, 1, 1000, PH, PW, sr) == 0
+
+
+@pytest.mark.parametrize("limit", sorted(cases.QUAD_LIMITS))
+def test_quad_strip_dispatch_limits(limit, lib_option):
+    lib = _lib.load()
+    lib_option("B200_ROI_ALIGN_PATH", "quad")
+    ok, bad = cases.QUAD_LIMITS[limit]
+    N, H, W, R, PH, PW, sr = ok
+    assert lib.b200_roi_align_workspace_bytes(N, R, H, W, PH, PW, sr) > 0
+    N, H, W, R, PH, PW, sr = bad
+    assert lib.b200_roi_align_workspace_bytes(N, R, H, W, PH, PW, sr) == 0
+    if limit == "axis_pw":                                       # the transposed grid of each side lands on the same side
+        assert lib.b200_roi_align_workspace_bytes(1, 64, 50, 68, 3, 16, 2) > 0
+        assert lib.b200_roi_align_workspace_bytes(1, 64, 50, 68, 17, 3, 2) == 0
 
 
 def test_product_package_never_imports_oracle():

@@ -12,6 +12,7 @@ import pytest
 import torch
 import torchvision
 
+from detectron.pytorch_b200 import synthetic as S
 from oracle import cpu as O
 from tests import cases
 
@@ -109,6 +110,61 @@ def test_roi_crop_equals_grid_sample():
     o.backward(torch.from_numpy(go))
     gi = O.roi_crop_backward(go, grid, img.shape, acc64=True)
     np.testing.assert_allclose(gi, rep_t.grad.numpy(), rtol=0, atol=1e-4)
+
+
+# Non-square pooled grids (PH, PW, sr): every kernel keeps separate PH / PW index arithmetic, and so must the oracle that
+# checks them -- a swap of the two sizes shows up as a wrong shape or as different values here.
+NON_SQUARE = [(7, 14, 2), (14, 7, 2), (3, 9, 1), (16, 5, 2), (1, 31, 1), (5, 3, 0)]
+
+
+def non_square_case(PH, PW, seed=0):
+    shape, scale = (2, 5, 38, 52), 1.0 / 8
+    f = S.make_features(shape, seed=seed)
+    r = np.concatenate([S.make_rois(28, shape, scale, seed=seed, min_size=8, max_size=400),
+                        S.make_edge_rois(shape, scale)]).astype(np.float32)
+    dy = np.random.RandomState(seed + 1).standard_normal((r.shape[0], shape[1], PH, PW)).astype(np.float32)
+    return shape, scale, f, r, dy
+
+
+@pytest.mark.parametrize("PH,PW,sr", NON_SQUARE)
+def test_roi_align_non_square_vs_torchvision(PH, PW, sr):
+    shape, scale, f, r, dy = non_square_case(PH, PW)
+    tv = torchvision.ops.roi_align(torch.from_numpy(f), torch.from_numpy(r), (PH, PW), scale, sr, aligned=False).numpy()
+    O.set_fused(False)
+    try:
+        out = O.roi_align_forward(f, r, PH, PW, scale, sr)
+    finally:
+        O.set_fused(True)
+    assert out.shape == (r.shape[0], shape[1], PH, PW)
+    assert np.array_equal(out, tv)                                         # bit-exact unfused
+    np.testing.assert_allclose(O.roi_align_forward(f, r, PH, PW, scale, sr), tv, rtol=0, atol=1e-4)
+    # backward vs torchvision's autograd in float64 (same sample positions: the RoIs are exact in float32)
+    ft = torch.from_numpy(f.astype(np.float64)).requires_grad_(True)
+    o = torchvision.ops.roi_align(ft, torch.from_numpy(r.astype(np.float64)), (PH, PW), scale, sr, aligned=False)
+    o.backward(torch.from_numpy(dy.astype(np.float64)))
+    dx = O.roi_align_backward(dy, r, shape, PH, PW, scale, sr, acc64=True)
+    np.testing.assert_allclose(dx, ft.grad.numpy(), rtol=0, atol=1e-4)
+    # the transposed grid is a different operation: a kernel that swaps PH and PW cannot pass both
+    if PH != PW:
+        tv_t = torchvision.ops.roi_align(torch.from_numpy(f), torch.from_numpy(r), (PW, PH), scale, sr, aligned=False).numpy()
+        assert not np.allclose(tv_t, np.swapaxes(out, 2, 3), atol=1e-3)
+
+
+@pytest.mark.parametrize("PH,PW", [(PH, PW) for PH, PW, _ in NON_SQUARE])
+def test_roi_pool_non_square_vs_torchvision(PH, PW):
+    shape, scale, f, r, dy = non_square_case(PH, PW)
+    out, argmax = O.roi_pool_forward(f, r, PH, PW, scale)
+    tv = torchvision.ops.roi_pool(torch.from_numpy(f), torch.from_numpy(r), (PH, PW), scale).numpy()
+    assert out.shape == (r.shape[0], shape[1], PH, PW)
+    assert np.array_equal(out, tv)
+    sel = argmax >= 0
+    assert np.array_equal(f.reshape(-1)[argmax[sel]], out[sel])
+    assert np.all(out[~sel] == 0)
+    # backward: where the reference's feasibility test keeps every contribution, the gradient is a scatter of dy at argmax
+    dx = O.roi_pool_backward(dy, argmax, r, shape, PH, PW, scale)
+    scat = np.zeros(f.size, np.float64)
+    np.add.at(scat, argmax[sel], dy[sel].astype(np.float64))
+    assert np.mean(np.abs(dx.reshape(-1) - scat) > 1e-4) < 0.01
 
 
 def _py_greedy_nms(b, thresh):
