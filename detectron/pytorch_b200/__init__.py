@@ -13,7 +13,7 @@ or, to make an unmodified checkout of the reference pick these up under ITS impo
 __version__ = "0.1.0"
 
 
-def install_reference_aliases(overwrite=True, proposals=False, nms=False):
+def install_reference_aliases(overwrite=True, proposals=False, nms=False, segm=False):
     """Register this package's op modules in sys.modules under the reference's import paths.
 
     After this, `from modeling.roi_xfrom.roi_align.functions.roi_align import RoIAlignFunction`
@@ -27,6 +27,9 @@ def install_reference_aliases(overwrite=True, proposals=False, nms=False):
     `nms=True` re-points the reference's `utils.boxes.nms` (lib/utils/boxes.py:320-324; called from
     generate_proposals.py:161 and core/test.py:764 with numpy arrays) at the device NMS (`utils/boxes.py` here); the
     reference's `utils.boxes` must be importable for that.
+    `segm=True` re-points the reference's `core.test.segm_results` (lib/core/test.py:793-847, called by im_detect_all)
+    at `core.test.segm_results` here, bound to the reference's `cfg`: the mask paste and RLE run on the device.  The
+    reference's `core.test` and `core.config` must be importable for that.
     """
     import importlib
     import sys
@@ -66,4 +69,10 @@ def install_reference_aliases(overwrite=True, proposals=False, nms=False):
         ref_boxes = importlib.import_module("utils.boxes")          # the reference's module
         ref_boxes.nms = importlib.import_module(__name__ + ".utils.boxes").nms
         installed.append("utils.boxes.nms")
+    if segm:
+        ref_test = importlib.import_module("core.test")             # the reference's module
+        ref_cfg = importlib.import_module("core.config").cfg
+        impl = importlib.import_module(__name__ + ".core.test").segm_results
+        ref_test.segm_results = lambda cls_boxes, masks, ref_boxes, im_h, im_w: impl(cls_boxes, masks, ref_boxes, im_h, im_w, cfg=ref_cfg)
+        installed.append("core.test.segm_results")
     return installed

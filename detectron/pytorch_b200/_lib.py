@@ -89,6 +89,15 @@ _SIGNATURES = {
     "b200_fast_rcnn_targets": (ctypes.c_int, [_c_float_p, _c_float_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
                                               ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_float,
                                               ctypes.c_void_p, _c_float_p, _c_float_p, _c_float_p, _c_float_p, _stream_t]),
+    # (masks, mask_channel, ref_boxes, D, K, M, im_h, im_w, thresh, out, stream)
+    "b200_segm_paste": (ctypes.c_int, [_c_float_p, ctypes.c_void_p, _c_float_p] + [ctypes.c_int] * 5 + [ctypes.c_float, ctypes.c_void_p,
+                                                                                                         _stream_t]),
+    # (masks, mask_channel, ref_boxes, D, K, M, im_h, im_w, thresh, offsets_out, stream)
+    "b200_segm_rle_count": (ctypes.c_int, [_c_float_p, ctypes.c_void_p, _c_float_p] + [ctypes.c_int] * 5 + [ctypes.c_float,
+                                                                                                             ctypes.c_void_p, _stream_t]),
+    # (masks, mask_channel, ref_boxes, D, K, M, im_h, im_w, thresh, offsets, runs_out, stream)
+    "b200_segm_rle_emit": (ctypes.c_int, [_c_float_p, ctypes.c_void_p, _c_float_p] + [ctypes.c_int] * 5 + [ctypes.c_float, ctypes.c_void_p,
+                                                                                                            ctypes.c_void_p, _stream_t]),
 }
 
 EXPORTED_SYMBOLS = tuple(sorted(_SIGNATURES))

@@ -102,6 +102,10 @@ size_t nms_batched_workspace_bytes(const int*, int);
 int soft_nms_batched(float*, const int*, int, float, float, float, int, int*, int*, cudaStream_t);
 int box_voting_batched(const float*, const int*, const float*, const int*, int, float, int, float, float*, cudaStream_t);
 int nms_batched(const float*, const int*, int, int, float, int*, int*, void*, size_t, cudaStream_t);
+bool segm_args_ok(int, int, int, int, int);
+int segm_paste(const float*, const int*, const float*, int, int, int, int, int, float, unsigned char*, cudaStream_t);
+int segm_rle_count(const float*, const int*, const float*, int, int, int, int, int, float, long long*, cudaStream_t);
+int segm_rle_emit(const float*, const int*, const float*, int, int, int, int, int, float, const long long*, int*, cudaStream_t);
 size_t roi_align_bwd_nhwc_workspace_bytes(int, int, int, int);
 int roi_align_backward_nhwc(const float*, float, int, int, int, int, int, int, int, int, const float*, float*, const int*, void*, size_t, cudaStream_t);
 
@@ -550,6 +554,32 @@ int b200_fast_rcnn_targets(const float* boxes_dev, const float* gt_boxes_dev, co
     return fast_rcnn_targets(boxes_dev, gt_boxes_dev, argmax_dev, max_classes_dev, keep_inds_dev, num_keep, num_fg, bbox_reg_weights_host,
                              num_reg_classes, cls_agnostic, im_scale, batch_idx, labels_out_dev, rois_out_dev, bbox_targets_out_dev,
                              inside_weights_out_dev, outside_weights_out_dev, (cudaStream_t)stream);
+}
+
+// test-time mask paste (N3, masks): lib/core/test.py:793-847, lib/utils/boxes.py:233-249 (expand_boxes)
+int b200_segm_paste(const float* masks_dev, const int* mask_channel_dev, const float* ref_boxes_dev, int num_dets, int num_channels,
+                    int resolution, int im_h, int im_w, float thresh, unsigned char* masks_out_dev, b200_stream_t stream) {
+    if (!segm_args_ok(num_dets, num_channels, resolution, im_h, im_w)) return B200_ROI_EINVAL;
+    if (num_dets > 0 && (!masks_dev || !ref_boxes_dev || !masks_out_dev)) return B200_ROI_EINVAL;
+    return segm_paste(masks_dev, mask_channel_dev, ref_boxes_dev, num_dets, num_channels, resolution, im_h, im_w, thresh, masks_out_dev,
+                      (cudaStream_t)stream);
+}
+
+int b200_segm_rle_count(const float* masks_dev, const int* mask_channel_dev, const float* ref_boxes_dev, int num_dets, int num_channels,
+                        int resolution, int im_h, int im_w, float thresh, long long* offsets_out_dev, b200_stream_t stream) {
+    if (!segm_args_ok(num_dets, num_channels, resolution, im_h, im_w)) return B200_ROI_EINVAL;
+    if (num_dets > 0 && (!masks_dev || !ref_boxes_dev || !offsets_out_dev)) return B200_ROI_EINVAL;
+    return segm_rle_count(masks_dev, mask_channel_dev, ref_boxes_dev, num_dets, num_channels, resolution, im_h, im_w, thresh,
+                          offsets_out_dev, (cudaStream_t)stream);
+}
+
+int b200_segm_rle_emit(const float* masks_dev, const int* mask_channel_dev, const float* ref_boxes_dev, int num_dets, int num_channels,
+                       int resolution, int im_h, int im_w, float thresh, const long long* offsets_dev, int* runs_out_dev,
+                       b200_stream_t stream) {
+    if (!segm_args_ok(num_dets, num_channels, resolution, im_h, im_w)) return B200_ROI_EINVAL;
+    if (num_dets > 0 && (!masks_dev || !ref_boxes_dev || !offsets_dev || !runs_out_dev)) return B200_ROI_EINVAL;
+    return segm_rle_emit(masks_dev, mask_channel_dev, ref_boxes_dev, num_dets, num_channels, resolution, im_h, im_w, thresh, offsets_dev,
+                         runs_out_dev, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -505,3 +505,54 @@ def nms_raw(dets, thresh):
                                 ws.data_ptr(), ws_bytes, _stream()),
                    "b200_nms")
     return keep, num_out
+
+
+# ------------------------------------------------------------------------------------------------
+# Test-time mask paste (lib/core/test.py:793-847 segm_results)
+# ------------------------------------------------------------------------------------------------
+def _segm_args(masks, mask_channel, ref_boxes, im_h, im_w):
+    _need_cuda_f32(masks, "masks"); _need_cuda_f32(ref_boxes, "ref_boxes")
+    if masks.dim() != 4 or masks.size(2) != masks.size(3):
+        raise ValueError("masks must be (D, K, M, M), got %s" % (tuple(masks.shape),))
+    D = masks.size(0)
+    if tuple(ref_boxes.shape) != (D, 4):
+        raise ValueError("ref_boxes must be (D, 4) = [x1, y1, x2, y2], got %s" % (tuple(ref_boxes.shape),))
+    if mask_channel is None:
+        chan = None
+    else:
+        chan = torch.as_tensor(mask_channel, dtype=torch.int32, device=masks.device).reshape(-1).contiguous()
+        if chan.numel() != D:
+            raise ValueError("mask_channel must hold one channel per detection (%d), got %d" % (D, chan.numel()))
+    return masks.contiguous(), chan, ref_boxes.contiguous(), D, masks.size(1), masks.size(2), int(im_h), int(im_w)
+
+
+def segm_paste(masks, mask_channel, ref_boxes, im_h, im_w, thresh=0.5):
+    """Dense binary masks (D, im_h, im_w) uint8 on the device: detection i's soft mask masks[i, mask_channel[i]]
+    (None: channel 0) resized to its (M + 2) / M-expanded box like cv2.resize with IPP off, `> thresh`, pasted into the
+    image (lib/core/test.py:806-833)."""
+    masks, chan, boxes, D, K, M, im_h, im_w = _segm_args(masks, mask_channel, ref_boxes, im_h, im_w)
+    out = torch.empty((D, im_h, im_w), dtype=torch.uint8, device=masks.device)
+    with torch.cuda.device(masks.device):
+        _lib.check(_lib.load().b200_segm_paste(masks.data_ptr(), chan.data_ptr() if chan is not None else None, boxes.data_ptr(), D, K, M,
+                                               im_h, im_w, float(thresh), out.data_ptr(), _stream()), "b200_segm_paste")
+    return out
+
+
+def segm_rle(masks, mask_channel, ref_boxes, im_h, im_w, thresh=0.5):
+    """COCO uncompressed RLE of the masks segm_paste would produce, without materialising them.  Returns host numpy
+    arrays (runs int32, counts int64): detection i's run lengths are runs[sum(counts[:i]) : sum(counts[:i + 1])],
+    column-major, alternating from a run of zeros.  One host read of the counts, one copy of all runs."""
+    import numpy as np
+    masks, chan, boxes, D, K, M, im_h, im_w = _segm_args(masks, mask_channel, ref_boxes, im_h, im_w)
+    if D == 0:
+        return np.zeros((0,), np.int32), np.zeros((0,), np.int64)
+    lib = _lib.load()
+    args = (masks.data_ptr(), chan.data_ptr() if chan is not None else None, boxes.data_ptr(), D, K, M, im_h, im_w, float(thresh))
+    offsets = torch.empty((D + 1,), dtype=torch.int64, device=masks.device)
+    with torch.cuda.device(masks.device):
+        _lib.check(lib.b200_segm_rle_count(*args, offsets.data_ptr(), _stream()), "b200_segm_rle_count")
+        offs = offsets.cpu().numpy()
+        runs = torch.empty((max(int(offs[-1]), 1),), dtype=torch.int32, device=masks.device)
+        _lib.check(lib.b200_segm_rle_emit(*args, offsets.data_ptr(), runs.data_ptr(), _stream()), "b200_segm_rle_emit")
+        runs_h = runs[:int(offs[-1])].cpu().numpy()
+    return runs_h, np.diff(offs).astype(np.int64)

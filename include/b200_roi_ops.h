@@ -219,6 +219,33 @@ B200_API int b200_box_voting_batched(const float* top_dets_dev, const int* top_c
                                      const int* all_counts_host, int num_problems, float thresh, int scoring_method, float beta,
                                      float* out_dev, b200_stream_t stream);
 
+/* ---- test-time mask paste (N3, masks) ----------------------------------------------------------------------------
+ * replaces the per-detection host loop of segm_results, lib/core/test.py:793-847, with expand_boxes,
+ * lib/utils/boxes.py:233-249 (cv2.resize + threshold + paste + pycocotools RLE encode).
+ * Detection i: soft mask = channel mask_channel[i] of masks (num_dets, num_channels, resolution, resolution) fp32
+ * (mask_channel: int32 device array, NULL = channel 0 for every detection; a channel outside [0, num_channels) gives an
+ * empty mask); ref_boxes (num_dets, 4) fp32 (x1, y1, x2, y2) in image pixels.  The box is expanded by
+ * (resolution + 2) / resolution in float32 and truncated to int32, the zero-padded mask is resized to it exactly like
+ * cv2.resize(INTER_LINEAR) on float32 with IPP disabled, binarised with `value > thresh` and pasted into the box's window
+ * clipped to the im_h x im_w image.  Limits: resolution <= 126, im_w <= 32768, im_h * im_w < 2^31, else B200_ROI_EINVAL.
+ * b200_segm_paste      masks_out (num_dets, im_h, im_w) uint8, every byte written (1 inside the mask, 0 elsewhere).
+ * b200_segm_rle_count  offsets_out: int64[num_dets + 1], the exclusive scan of the number of runs of each detection's
+ *                      COCO uncompressed RLE (column-major image, run lengths alternating from a run of zeros, which
+ *                      is 0 when pixel (0, 0) is set; they sum to im_h * im_w); offsets_out[num_dets] is the total.
+ * b200_segm_rle_emit   runs_out: int32[offsets[num_dets]]; detection i's runs at runs_out + offsets[i].  `offsets` is
+ *                      b200_segm_rle_count's output for the same arguments.
+ * Each entry point launches a fixed number of kernels whatever num_dets is (paste 1, count 2, emit 1), none for
+ * num_dets == 0. */
+B200_API int b200_segm_paste(const float* masks_dev, const int* mask_channel_dev, const float* ref_boxes_dev, int num_dets,
+                             int num_channels, int resolution, int im_h, int im_w, float thresh, unsigned char* masks_out_dev,
+                             b200_stream_t stream);
+B200_API int b200_segm_rle_count(const float* masks_dev, const int* mask_channel_dev, const float* ref_boxes_dev, int num_dets,
+                                 int num_channels, int resolution, int im_h, int im_w, float thresh, long long* offsets_out_dev,
+                                 b200_stream_t stream);
+B200_API int b200_segm_rle_emit(const float* masks_dev, const int* mask_channel_dev, const float* ref_boxes_dev, int num_dets,
+                                int num_channels, int resolution, int im_h, int im_w, float thresh, const long long* offsets_dev,
+                                int* runs_out_dev, b200_stream_t stream);
+
 /* ---- introspection used by the benchmark / tests (no compute) ----------------------------------
  * Number of kernel launches the library has enqueued since load (all entry points). */
 B200_API unsigned long long b200_roi_ops_launch_count(void);
